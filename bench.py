@@ -2,6 +2,7 @@
 """bench.py — images/sec of one MobileNetV2-1.0 224x224 training step (BASELINE.json metric).
 
   python bench.py --gpus N --steps K --warmup W            # this repo's sm_100a path
+  python bench.py ... --dump-outputs DIR                    # + the last timed step's outputs (.npy)
   python bench.py --impl reference --gpus N --steps K ...   # the reference's CPU path (port)
   python bench.py --impl torch_gpu --steps K ...            # context: the reference's stock-torch
                                                             # graph (cuDNN/ATen) on the same B200
@@ -267,7 +268,7 @@ def run_torch_gpu(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    ctx = torch_gpu_context(args.batch, steps=max(3, min(args.steps, 10)),
+    ctx = torch_gpu_context(args.batch, steps=args.steps,
                             warmup=max(3, min(args.warmup, 5)), config=args.config)
     best = ctx["autocast_bf16_channels_last"]
     print(json.dumps({
@@ -337,6 +338,55 @@ def profile_kernels(ts, n_steps=2):
     return agg, total_ms / n_steps
 
 
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def flat_state(ts):
+    """The fp32 master weights (named_parameters order) and the BatchNorm running statistics
+    (named_buffers order), each as one flat copy."""
+    import torch
+    return (torch.cat([p.detach().flatten() for _, p in ts.model.named_parameters()]),
+            torch.cat([b.detach().flatten() for b in ts.stat_bufs]))
+
+
+def train_state(ts):
+    """Every device tensor a training step reads and updates besides its scratch: the optimizer's
+    flat arenas (fp32 masters, bf16 mirror, RMSprop and EMA state), the model's buffers (BatchNorm
+    statistics) and their EMA shadows."""
+    A = ts.opt.arenas()
+    return [A[k] for k in ("p", "bf16", "sq", "mom", "gavg", "ema") if A[k] is not None] + \
+        list(ts.model.buffers()) + list(ts.stat_shadow)
+
+
+def dump_outputs(ts, out_dir, before):
+    """Write what TrainStep hands its caller after a step, as float32 DIR/<name>.npy: the
+    loss and top-1 / top-5 fractions of that step, the fp32 master weights and their EMA shadows
+    (flattened in named_parameters order), the BatchNorm running statistics and their EMA shadows
+    (flattened in named_buffers order), and the step's change of the weights and of the statistics
+    against `before` (flat_state() of the state the step started from; after one step from the
+    initial state both are dominated by their initial values, the changes are not).  If all of it
+    exceeds DUMP_BYTES, an array longer than an
+    equal share keeps a fixed sample of that many elements (numpy default_rng(0), indices
+    ascending), the same in every run."""
+    import numpy as np
+    import torch
+    params, stats = flat_state(ts)
+    out = {"loss": ts.loss, "top1": ts.top1, "top5": ts.top5, "params": params,
+           "params_ema": torch.cat([ts.opt.ema_shadow(p).flatten()
+                                    for _, p in ts.model.named_parameters()]),
+           "bn_stats": stats,
+           "bn_stats_ema": torch.cat([b.flatten() for b in ts.stat_shadow]),
+           "params_update": params - before[0], "bn_stats_update": stats - before[1]}
+    out = {k: t.detach().float().cpu().numpy() for k, t in out.items()}
+    room = (DUMP_BYTES - 4096 * len(out)) // 4                 # elements; 4 KB per .npy header
+    cap = room if sum(a.size for a in out.values()) <= room else room // len(out)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        if a.size > cap:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def load_peaks():
     p = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(p):
@@ -370,6 +420,9 @@ def run_ours(args):
         for t in model.state_dict().values():
             dist.broadcast(t, 0)
     ts = TrainStep(model, B)
+    # --dump-outputs: the state before the first step, the same in every run (seeded model)
+    start = [t.clone() for t in train_state(ts)] if args.dump_outputs else None
+    before = flat_state(ts) if args.dump_outputs else None
     g = torch.Generator().manual_seed(rank)
     host = []
     for i in range(2):
@@ -399,11 +452,26 @@ def run_ours(args):
     launches0 = engine.LAUNCHES
     sync_all()
     e0.record()
-    for _ in range(args.steps):
+    for _ in range(args.steps - (1 if start is not None else 0)):
         ts.run()
     e1.record()
+    if start is not None:
+        # The last timed step starts from `start` again: the order-dependent fp32 weight-gradient
+        # reductions differ in the last bits from run to run and the steps before amplify that, so
+        # only a step from a fixed state computes the same outputs in every run.  The copies sit
+        # between the two timed windows.
+        for t, s in zip(train_state(ts), start):
+            t.copy_(s)
+        ts.global_step = 0
+        e4, e5 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e4.record()
+        ts.run()
+        e5.record()
     sync_all()
-    ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
+    if start is not None and rank == 0:
+        dump_outputs(ts, args.dump_outputs, before)
+    ms = e0.elapsed_time(e1) + (e4.elapsed_time(e5) if start is not None else 0.0)
+    ms = torch.tensor([ms], device=dev)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms_total = float(ms)
@@ -542,7 +610,18 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-gpu-context", action="store_true",
                     help="skip the stock-PyTorch-on-this-GPU context measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (loss, top-1/5, "
+                         "weights, EMA shadows, BatchNorm statistics, the step's change of weights "
+                         "and statistics) as DIR/<name>.npy; that "
+                         "last timed step starts from the seeded state before the first step, so "
+                         "with the same arguments its inputs and outputs are the same in every run "
+                         "up to rounding and two builds compare file by file")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of this repo's path (--impl ours)")
     if args.batch is None:
         args.batch = CONFIGS[args.config][1]
     if args.impl == "reference":

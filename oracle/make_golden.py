@@ -1,7 +1,9 @@
 """ORACLE tooling — generates tests/golden/*.pt by running the LIVE reference
 (/root/reference, imported unmodified) on seeded inputs.  Run in the build container only:
 
-    python oracle/make_golden.py
+    python oracle/make_golden.py            # blocks.pt, optim.pt
+    python oracle/make_golden.py --nl       # blocks_nl.pt
+    python oracle/make_golden.py --step     # ref_step.pt
 
 The fixtures travel to the GPU box; /root/reference does not.
 Reference entry points exercised:
@@ -105,6 +107,92 @@ def main_nl():
     blocks = _block_records(mb, NL_CASES, {"momentum": 0.01, "eps": 1e-3})
     torch.save(blocks, os.path.join(OUT, "blocks_nl.pt"))
     print("blocks_nl.pt", os.path.getsize(os.path.join(OUT, "blocks_nl.pt")), "bytes")
+
+
+STEP_ROWS = [[1, 16, 1, 1, [3]], [6, 24, 1, 2, [3]], [6, 32, 1, 2, [3, 5]], [3, 40, 1, 2, [5]],
+             [3, 48, 2, 2, [3]]]
+STEP_KW = dict(inverted_residual_setting=STEP_ROWS, active_fn="nn.ReLU", batch_norm_momentum=0.01,
+               batch_norm_epsilon=1e-3, input_size=64, num_classes=10, last_channel=64)
+
+
+def _digest(tensors, k, g):
+    """Per named tensor: a tensor of at most one dimension in full (fp32); a larger one as float64
+    sum, sum of |x| and sum of x^2 of every output channel (dim 0) plus `k` elements at seeded flat
+    indices.  Everything is concatenated in `names` order; `count` splits the samples."""
+    names = list(tensors)
+    full, ch_sum, ch_abs, ch_sq, idx, val, count = [], [], [], [], [], [], []
+    for n in names:
+        t = tensors[n].detach()
+        if t.dim() <= 1:
+            full.append(t.float().flatten())
+            continue
+        rows = t.double().flatten(1)
+        ch_sum.append(rows.sum(1))
+        ch_abs.append(rows.abs().sum(1))
+        ch_sq.append(rows.square().sum(1))
+        v = t.float().flatten()
+        i = torch.randperm(v.numel(), generator=g)[:k].sort().values
+        idx.append(i.to(torch.int32))
+        val.append(v[i])
+        count.append(len(i))
+    return {"names": names, "numel": torch.tensor([tensors[n].numel() for n in names]),
+            "full": torch.cat(full), "ch_sum": torch.cat(ch_sum), "ch_abs": torch.cat(ch_abs),
+            "ch_sq": torch.cat(ch_sq), "count": torch.tensor(count), "idx": torch.cat(idx),
+            "val": torch.cat(val)}
+
+
+def main_step(k=64):
+    """tests/golden/ref_step.pt: three training steps of the reference (train.py:64-114 with the
+    live model, RMSprop, label-smoothed CE, 'mnas' L2 and EMA classes) on a small MobileNetV2 at
+    64x64, dropout off.  Per step the loss and a few input values (to pin the seeded batches);
+    after the last step every tensor of the state_dict and every EMA shadow as _digest()."""
+    sys.path.insert(0, REF)
+    warnings.simplefilter("ignore")
+    import models.mobilenet_base as rmb
+    import models.mobilenet_supernet as rsup
+    from utils.rmsprop import RMSprop
+    from utils import optim as roptim
+    B, steps, seed, data_seed = 8, 3, 1995, 0
+    torch.manual_seed(seed)
+    ref = rsup.Model(**STEP_KW)
+    ref.apply(rmb.init_weights_mnas)
+    for m in ref.modules():
+        if isinstance(m, torch.nn.Dropout):
+            m.p = 0.0
+    opt = RMSprop(ref.parameters(), lr=0.016 * B / 256, alpha=0.9, momentum=0.9, eps=1e-3,
+                  eps_inside_sqrt=True, weight_decay=0)
+    crit = roptim.CrossEntropyLabelSmooth(STEP_KW["num_classes"], 0.1)
+    ema = roptim.ExponentialMovingAverage(0.9999 ** (B / 4096.0))
+    for n, p in ref.named_parameters():
+        ema.register(n, p)
+    for n, b in ref.named_buffers():
+        if "running_var" in n or "running_mean" in n:
+            ema.register(n, b)
+    g = torch.Generator().manual_seed(data_seed)
+    losses, x_head, targets = [], [], []
+    for step in range(1, steps + 1):
+        x = torch.randn(B, 3, STEP_KW["input_size"], STEP_KW["input_size"], generator=g)
+        t = torch.randint(0, STEP_KW["num_classes"], (B,), generator=g)
+        ref.train()
+        opt.zero_grad()
+        loss = crit(ref(x), t).mean() + roptim.cal_l2_loss(ref, 1e-5, "mnas")
+        loss.backward()
+        opt.step()
+        named = dict(ref.named_parameters())
+        named.update(dict(ref.named_buffers()))
+        for n in ema.average_names():
+            ema(n, named[n], step)
+        losses.append(float(loss))
+        x_head.append(x.flatten()[:16].clone())
+        targets.append(t.clone())
+    gs = torch.Generator().manual_seed(11)
+    rec = {"kw": STEP_KW, "batch": B, "steps": steps, "seed": seed, "data_seed": data_seed,
+           "losses": losses, "x_head": torch.stack(x_head), "targets": torch.stack(targets),
+           "state": _digest(ref.state_dict(), k, gs),
+           "ema": _digest({n: ema.average(n) for n in ema.average_names()}, k, gs)}
+    path = os.path.join(OUT, "ref_step.pt")
+    torch.save(rec, path)
+    print("ref_step.pt", os.path.getsize(path), "bytes")
 
 
 def main():
@@ -212,5 +300,7 @@ def main():
 if __name__ == "__main__":
     if "--nl" in sys.argv:          # separate process: FLAGS of the reference is a singleton
         main_nl()
+    elif "--step" in sys.argv:
+        main_step()
     else:
         main()

@@ -15,8 +15,8 @@ not exist) and that serves as the end-to-end parity reference for the full netwo
 `as_reference(model)` deep-copies a model built from the package's boundary modules (identical
 module tree / state_dict to the reference's) and rebinds the two block classes' forward to the
 reference's stock-torch graph, so it runs on CPU (or on a GPU through cuDNN/ATen: the
-"stock PyTorch eager" context row).  Validated against the live reference by
-tests/test_oracle_step_vs_reference.py (runs only where /root/reference exists).
+"stock PyTorch eager" context row).  Validated against three steps of the live reference
+(oracle/make_golden.py --step -> tests/golden/ref_step.pt) by tests/test_oracle_step_vs_reference.py.
 """
 import copy
 import types

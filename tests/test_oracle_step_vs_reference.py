@@ -1,70 +1,68 @@
-"""CPU, build container only: pin oracle/torch_model.py (the CPU-baseline port of the whole
-training step) against the LIVE reference classes.  Skipped where /root/reference is absent."""
+"""CPU: pin oracle/torch_model.py (the CPU-baseline port of the whole training step) against three
+training steps of the reference's own model, RMSprop, loss, L2 and EMA classes, recorded by
+oracle/make_golden.py --step in tests/golden/ref_step.pt: the losses, every one-dimensional tensor
+in full and every output channel of the larger ones."""
 import os
-import sys
 import warnings
 
-import pytest
 import torch
 
-REF = os.environ.get("YAMB_REFERENCE", "/root/reference")
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "models")),
-                                reason="reference tree not present (GPU box)")
 
-ROWS = [[1, 16, 1, 1, [3]], [6, 24, 1, 2, [3]], [6, 32, 1, 2, [3, 5]], [3, 40, 1, 2, [5]],
-        [3, 48, 2, 2, [3]]]
-KW = dict(inverted_residual_setting=ROWS, active_fn="nn.ReLU", batch_norm_momentum=0.01,
-          batch_norm_epsilon=1e-3, input_size=64, num_classes=10, last_channel=64)
+def _check(got, rec, what, rtol=1e-5, atol=1e-6):
+    """`got` (name -> tensor) against a record of oracle.make_golden._digest: tensors of at most one
+    dimension elementwise; larger ones on their seeded elements, and per output channel the sum and
+    the sum of squares within the bounds that elementwise closeness (|x - y| <= atol + rtol |y|)
+    implies."""
+    assert sorted(got) == sorted(rec["names"]), what
+    idx = iter(rec["idx"].long().split(rec["count"].tolist()))
+    val = iter(rec["val"].split(rec["count"].tolist()))
+    f = c = 0                                   # cursors into "full" and the per-channel sums
+    for j, n in enumerate(rec["names"]):
+        t = got[n].detach()
+        assert t.numel() == int(rec["numel"][j]), (what, n)
+        if t.dim() <= 1:
+            want = rec["full"][f:f + t.numel()]
+            f += t.numel()
+            assert torch.allclose(t.float().flatten(), want, rtol=rtol, atol=atol), (what, n)
+            continue
+        assert torch.allclose(t.float().flatten()[next(idx)], next(val), rtol=rtol, atol=atol), \
+            (what, n)
+        rows = t.double().flatten(1)
+        k = rows.shape[1]
+        s1, s2 = rec["ch_abs"][c:c + len(rows)], rec["ch_sq"][c:c + len(rows)]
+        d_sum = (rows.sum(1) - rec["ch_sum"][c:c + len(rows)]).abs()
+        d_sq = (rows.square().sum(1) - s2).abs()
+        c += len(rows)
+        bad_sum = (d_sum > atol * k + rtol * s1).nonzero().flatten().tolist()
+        bad_sq = (d_sq > atol * atol * k + 2 * atol * (1 + rtol) * s1 + (2 * rtol + rtol * rtol) * s2)
+        assert not bad_sum and not bad_sq.any(), (what, n, "channels", bad_sum,
+                                                 bad_sq.nonzero().flatten().tolist())
+    assert f == rec["full"].numel() and c == rec["ch_sum"].numel(), what
 
 
-def test_port_step_equals_reference_step():
-    sys.path.insert(0, REF)
+def test_port_step_equals_reference_step(golden_dir):
     warnings.simplefilter("ignore")
-    import models.mobilenet_base as rmb
-    import models.mobilenet_supernet as rsup
-    from utils.rmsprop import RMSprop
-    from utils import optim as roptim
     from yet_another_mobilenet_series_b200 import mobilenet_base as mb, mobilenet_supernet as sup
     from oracle import torch_model as tm
 
-    torch.manual_seed(1995)
-    ref = rsup.Model(**KW)
-    ref.apply(rmb.init_weights_mnas)
-    torch.manual_seed(1995)
-    ours = sup.Model(**KW)
+    rec = torch.load(os.path.join(golden_dir, "ref_step.pt"), weights_only=False)
+    kw, B = rec["kw"], rec["batch"]
+    torch.manual_seed(rec["seed"])
+    ours = sup.Model(**kw)
     ours.apply(mb.init_weights_mnas)
     port = tm.as_reference(ours)
-    for m in list(ref.modules()) + list(port.modules()):
+    for m in port.modules():
         if isinstance(m, torch.nn.Dropout):
             m.p = 0.0
-    B = 8
     trainer = tm.RefTrainer(port, B)
-    opt = RMSprop(ref.parameters(), lr=0.016 * B / 256, alpha=0.9, momentum=0.9, eps=1e-3,
-                  eps_inside_sqrt=True, weight_decay=0)
-    crit = roptim.CrossEntropyLabelSmooth(10, 0.1)
-    ema = roptim.ExponentialMovingAverage(0.9999 ** (B / 4096.0))
-    for n, p in ref.named_parameters():
-        ema.register(n, p)
-    for n, b in ref.named_buffers():
-        if "running_var" in n or "running_mean" in n:
-            ema.register(n, b)
-    g = torch.Generator().manual_seed(0)
-    for step in range(1, 4):
-        x = torch.randn(B, 3, 64, 64, generator=g)
-        t = torch.randint(0, 10, (B,), generator=g)
-        ref.train()
-        opt.zero_grad()
-        loss = crit(ref(x), t).mean() + roptim.cal_l2_loss(ref, 1e-5, "mnas")
-        loss.backward()
-        opt.step()
-        named = dict(ref.named_parameters())
-        named.update(dict(ref.named_buffers()))
-        for n in ema.average_names():
-            ema(n, named[n], step)
+    g = torch.Generator().manual_seed(rec["data_seed"])
+    for step in range(rec["steps"]):
+        x = torch.randn(B, 3, kw["input_size"], kw["input_size"], generator=g)
+        t = torch.randint(0, kw["num_classes"], (B,), generator=g)
+        assert torch.equal(x.flatten()[:16], rec["x_head"][step])   # the recorded batches
+        assert torch.equal(t, rec["targets"][step])
         lp = trainer.step(x, t)
-        assert abs(lp - float(loss)) < 1e-5 * max(1.0, abs(float(loss)))
-    sa, sb = ref.state_dict(), port.state_dict()
-    for k in sa:
-        assert torch.allclose(sa[k].float(), sb[k].float(), rtol=1e-5, atol=1e-6), k
-    for n in ema.average_names():
-        assert torch.allclose(ema.average(n), trainer.ema.shadow[n], rtol=1e-5, atol=1e-6), n
+        want = rec["losses"][step]
+        assert abs(lp - want) < 1e-5 * max(1.0, abs(want)), (step, lp, want)
+    _check({k: v.float() for k, v in port.state_dict().items()}, rec["state"], "state_dict")
+    _check(trainer.ema.shadow, rec["ema"], "EMA shadow")
